@@ -6,6 +6,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...     # the reference's CPU fbgemm path on the host cores
+    python bench.py ... --dump-outputs DIR   # also write the last timed step's logits to DIR/logits.npy
 
 A step is one forward pass of the hot path over one synthetic batch per rank.  `value` is timed with
 the inputs already resident in HBM; `e2e` goes through the reference-facing call with HOST buffers
@@ -145,6 +146,15 @@ def build_reference_module(workload: str):
     return mf.cast_fp16(mf.make_teacher())
 
 
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """`--dump-outputs`: each array as <out_dir>/<name>.npy in float32, so that two builds (or the two arms) run with the
+    same arguments can be compared output for output.  The inputs are seeded, hence identical from run to run."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.detach().float().cpu().numpy())
+
+
 def peaks():
     path = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(path):
@@ -217,7 +227,8 @@ def layer_table(net, n, fused_front=True):
 
 
 def _reference_forward_times(workload: str, bs: int, warmup: int, steps: int):
-    """Seconds per forward of the reference's own CPU path (torch fbgemm / CPU half) on all host threads."""
+    """Seconds per forward of the reference's own CPU path (torch fbgemm / CPU half) on all host threads, and the logits
+    of the last forward."""
     from ievm_b200 import synthetic as mf
     torch.set_num_threads(os.cpu_count() or 1)
     gm = build_reference_module(workload)
@@ -232,15 +243,15 @@ def _reference_forward_times(workload: str, bs: int, warmup: int, steps: int):
             gm(x)
         for _ in range(steps):
             t0 = time.perf_counter()
-            gm(x)
+            y = gm(x)
             times.append(time.perf_counter() - t0)
-    return times
+    return times, y
 
 
 def cpu_baseline_sample(workload: str, bs: int):
     """The reference's own CPU path on the host cores, bounded sample: 1 warm-up + 5 forwards of the headline batch
     (about 1-2 s of CPU work at ~1.6 k img/s), median step."""
-    times = sorted(_reference_forward_times(workload, bs, 1, 5))
+    times = sorted(_reference_forward_times(workload, bs, 1, 5)[0])
     med = times[len(times) // 2]
     return {"value": bs / med, "unit": "images/s", "cores": torch.get_num_threads(), "kind": "port",
             "sample": f"median of {len(times)} forwards of batch {bs} through torch's fbgemm/ATen CPU path (the module "
@@ -254,7 +265,9 @@ def run_reference(args, rank, world):
     if rank != 0:
         return
     bs = args.ref_batch or args.batch
-    times = _reference_forward_times(args.workload, bs, args.warmup, args.steps)
+    times, y = _reference_forward_times(args.workload, bs, args.warmup, args.steps)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logits": y})
     med = sorted(times)[len(times) // 2]
     val = bs / med
     desc, dtype = WORKLOADS[args.workload]
@@ -458,6 +471,9 @@ def run_b200(args, rank, world, local_rank):
 
     # ---- logits gathered over NVLink for reporting; the gather must equal a single-GPU run of the same images ----
     gathered = gather_logits(y.float(), world * n, rank, world)
+    if rank == 0 and args.dump_outputs:
+        # the logits of the last timed step, every rank's shard in batch order (24 bytes per image)
+        dump_outputs(args.dump_outputs, {"logits": gathered})
     gather_bitexact = None
     if world > 1:
         ok = True
@@ -647,7 +663,11 @@ def main():
     ap.add_argument("--no-latency", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip strong scaling and the secondary workloads")
     ap.add_argument("--latency-runs", type=int, default=300)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the logits of the last one to DIR/logits.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
