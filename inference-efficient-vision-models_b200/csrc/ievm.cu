@@ -1779,9 +1779,13 @@ int ievm_create(const ievm_net_desc* nd, int device, int max_batch, ievm_handle*
     for (size_t i = 0; i < h->layers.size(); ++i) {
       const LayerPlan& L = h->layers[i];
       if (L.d.op != IEVM_OP_CONV || L.is_stem) continue;
-      fprintf(stderr, "[ievm] layer %2zu %dx%d s%d %4d->%4d @%dx%d mode=%s kc=%d kchunks=%d bn=%d n_tiles=%d cluster=%d stages=%d kb_group=%d band=%dx%d rows residentB=%d fast_round=%d smem=%zu\n",
+      // dual: the form of the launch this conv rides in (both convs of a pair print it); subs: halo sub-tiles per image
+      const LayerPlan& P = L.dual_of >= 0 ? h->layers[L.dual_of] : L;
+      const char* dual = P.dual_partner < 0 ? "none" : P.dual_s2 ? "s2" : P.dual_wide ? "wide" : "plain";
+      fprintf(stderr, "[ievm] layer %2zu %dx%d s%d %4d->%4d @%dx%d mode=%s kc=%d kchunks=%d bn=%d n_tiles=%d cluster=%d stages=%d kb_group=%d band=%dx%d rows residentB=%d fast_round=%d smem=%zu two_cta=%d dual=%s zcorr=%d subs=%d\n",
               i, L.d.ksize, L.d.ksize, L.d.stride, L.d.cin, L.d.cout, L.ho, L.wo, L.mode == kModeHalo ? "halo" : "im2col",
-              L.kc_bytes, L.kchunks, L.bn, L.n_tiles, L.cluster, L.stages, L.kb_group, L.band_subs, L.sub_rows, L.resident_b, L.fast_round, L.smem_bytes);
+              L.kc_bytes, L.kchunks, L.bn, L.n_tiles, L.cluster, L.stages, L.kb_group, L.band_subs, L.sub_rows, L.resident_b, L.fast_round, L.smem_bytes,
+              L.two_cta, dual, L.zcorr != nullptr ? 1 : 0, L.subs_per_img);
     }
   }
   if (rc == IEVM_OK) rc = assign_buffers(h);

@@ -329,31 +329,17 @@ def test_kernel_configuration_fallbacks_stay_bit_exact(env, tmp_path):
 def test_tensor_core_convs_with_nonzero_input_zero_points():
     """SURVEY section 7: a tensor-core layer whose input zero point is not 0 gets the border-aware -zp * sum(w)
     correction instead of being refused.  The converted ResNet never has one (every conv input is post-ReLU), so the
-    test moves the zero points of block outputs and of the ConvReLU2d outputs away from 0 in BOTH the oracle's network
-    and the engine's flattened description, and demands bit-exact tensors and accumulators again -- through the
-    halo kernel (layers 1-2), the im2col kernels (stride 2, 1x1, layers 3-4), the CTA-pair kernels and the head."""
-    import copy
+    test moves the zero points of block outputs and of the ConvReLU2d outputs away from 0 in the converted module
+    (tests/ievm_testutil.py: with_nonzero_zero_points), so the oracle and the engine's flattened description both read
+    them, and demands bit-exact tensors and accumulators again -- through the halo kernel (layers 1-2), the im2col
+    kernels (stride 2, 1x1, layers 3-4), the CTA-pair kernels and the head."""
     import ievm_b200
-    gm = cached_quantized(mf.PRUNED_WIDTHS)
-    onet = copy.deepcopy(O.extract_qnet(gm))
-    spec = copy.deepcopy(ievm_b200.from_converted(gm))
-    by_name = {L.name: L for L in spec.layers}
-    zp_of_tensor = {}
-    for bi, blk in enumerate(onet.blocks):
-        blk.conv1.out_zp = 3 + 2 * bi           # ReLU conv: values clamp at the zero point
-        blk.add_zp = 5 + 3 * bi                 # block output feeds the next block's conv1 / downsample / residual
-        li, bj = bi // 2 + 1, bi % 2
-        c1, c2 = by_name[f"layer{li}.{bj}.conv1"], by_name[f"layer{li}.{bj}.conv2"]
-        c1.out_zp = blk.conv1.out_zp
-        c2.add_zp = blk.add_zp
-        zp_of_tensor[c1.out_tensor] = c1.out_zp
-        zp_of_tensor[c2.out_tensor] = c2.add_zp
-    for L in spec.layers:                        # consumers read the producers' new zero points
-        if L.in_tensor in zp_of_tensor:
-            L.in_zp = zp_of_tensor[L.in_tensor]
-        if L.res_tensor in zp_of_tensor and f"{L.name}".endswith("conv2"):
-            L.res_zp = zp_of_tensor[L.res_tensor]
+    from ievm_testutil import with_nonzero_zero_points
+    gm = with_nonzero_zero_points(cached_quantized(mf.PRUNED_WIDTHS))
+    onet = O.extract_qnet(gm)
+    spec = ievm_b200.from_converted(gm)
     assert sum(1 for L in spec.layers if L.op == 0 and L.in_zp != 0 and L.in_tensor != 0) >= 15
+    assert [b.add_zp for b in onet.blocks] == [5 + 3 * i for i in range(8)]
     eng = ievm_b200.B200QuantizedResNet(spec, max_batch=8)
     eng.set_option("keep_tensors", 1)
     x = mf.synthetic_images(5, seed=33)
