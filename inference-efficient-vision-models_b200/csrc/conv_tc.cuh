@@ -252,6 +252,113 @@ __device__ __forceinline__ int round_add_max(float x, int zp, int lo) {
   return max(__float2int_rn(x) + zp, lo);
 }
 
+#ifndef IEVM_EXP_SCALAR_EPI
+// Paired forms (default): values 2j and 2j + 1 of a chunk go through one FADD2 / FMUL2 / FFMA2 (add/mul/fma.rn.f32x2),
+// each lane rounded exactly like the scalar op, so the arithmetic is the scalar definition's, op for op.
+//
+// Contraction fence: ptxas contracts mul.rn.f32x2 followed by add.rn.f32x2 into one FFMA2 although both carry .rn (it
+// never does this to scalar mul.rn / add.rn), also under -fmad=false.  fl(x * mu + M) differs from fl(fl(x * mu) + M)
+// whenever the exact product lies within half an ulp of a .5 point, so every multiply whose result feeds the
+// magic-number add is written as fma(x, mu, -0) instead: equal to fl(x * mu) for every input (+-0 + -0 keeps the sign of
+// a zero product, every other sum is the product), and an FFMA2 has nothing left to contract.  The -0 comes from the
+// constant bank, so ptxas cannot fold the fma back into a multiply; it is an FFMA2 operand (uniform register), and the
+// fence costs no instruction.
+__constant__ float2 g_neg_zero2 = {-0.0f, -0.0f};
+__device__ __forceinline__ float2 fmul2_fenced(float2 a, float2 b) { return __ffma2_rn(a, b, g_neg_zero2); }
+__device__ __forceinline__ float2 splat2(float a) { return make_float2(a, a); }
+__device__ __forceinline__ float2 i2f2(uint32_t a, uint32_t b) {
+  return make_float2(__int2float_rn(static_cast<int>(a)), __int2float_rn(static_cast<int>(b)));
+}
+
+// 16 accumulators -> 16 requantised bytes (no residual).
+template <bool kFast>
+__device__ __forceinline__ uint4 epilogue16_i8(const uint32_t (&v)[16], const float* s_bd, const float* s_mu, int zp,
+                                               int lo) {
+  int q[16];
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const float4 b4 = *reinterpret_cast<const float4*>(s_bd + 4 * j);
+    const float4 m4 = *reinterpret_cast<const float4*>(s_mu + 4 * j);
+    const float2 bd[2] = {make_float2(b4.x, b4.y), make_float2(b4.z, b4.w)};
+    const float2 mu[2] = {make_float2(m4.x, m4.y), make_float2(m4.z, m4.w)};
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const int i = 4 * j + 2 * h;
+      const float2 t = __fadd2_rn(i2f2(v[i], v[i + 1]), bd[h]);
+      if (kFast) {
+        const float2 u = __fadd2_rn(fmul2_fenced(t, mu[h]), splat2(kRoundMagic));
+        q[i] = __viaddmax_s32(__float_as_int(u.x), zp - kRoundMagicBits, lo);
+        q[i + 1] = __viaddmax_s32(__float_as_int(u.y), zp - kRoundMagicBits, lo);
+      } else {
+        const float2 u = __fmul2_rn(t, mu[h]);
+        q[i] = max(__float2int_rn(u.x) + zp, lo);
+        q[i + 1] = max(__float2int_rn(u.y) + zp, lo);
+      }
+    }
+  }
+  return make_uint4(pack4_sat_u8(q[0], q[1], q[2], q[3]), pack4_sat_u8(q[4], q[5], q[6], q[7]),
+                    pack4_sat_u8(q[8], q[9], q[10], q[11]), pack4_sat_u8(q[12], q[13], q[14], q[15]));
+}
+
+// 16 accumulators + 16 residual bytes -> 16 bytes of quantized::add_relu(requant(acc), residual).
+// All float steps reproduce the scalar definition exactly: clamping before rounding commutes with
+// RNE because the clamp bounds are integers, and (x + M) - M is RNE for |x| <= 256.
+template <bool kFast, bool kResI2F = false>
+__device__ __forceinline__ uint4 epilogue16_i8_res(const uint32_t (&v)[16], const uint4 r4, const float* s_bd,
+                                                   const float* s_mu, const AddReluConst& k) {
+  const uint32_t rw[4] = {r4.x, r4.y, r4.z, r4.w};
+  int q[16];
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const float4 b4 = *reinterpret_cast<const float4*>(s_bd + 4 * j);
+    const float4 m4 = *reinterpret_cast<const float4*>(s_mu + 4 * j);
+    const float2 bd[2] = {make_float2(b4.x, b4.y), make_float2(b4.z, b4.w)};
+    const float2 mu[2] = {make_float2(m4.x, m4.y), make_float2(m4.z, m4.w)};
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const int i = 4 * j + 2 * h;
+      float2 t = __fadd2_rn(i2f2(v[i], v[i + 1]), bd[h]);
+      // dequantised residual bytes 2h, 2h + 1 of the word (the two forms of float(byte): see the scalar form below)
+      const float2 rbyte =
+          kResI2F ? make_float2(static_cast<float>((rw[j] >> (16 * h)) & 0xffu), static_cast<float>((rw[j] >> (16 * h + 8)) & 0xffu))
+                  : __fadd2_rn(make_float2(__uint_as_float(__byte_perm(rw[j], 0x4B400000u, 0x7650 + 2 * h)),
+                                           __uint_as_float(__byte_perm(rw[j], 0x4B400000u, 0x7651 + 2 * h))),
+                               splat2(-kRoundMagic));
+      const float2 rb = __ffma2_rn(splat2(k.r_scale), rbyte, splat2(k.pb));
+      if (kFast) {
+        t = __fadd2_rn(fmul2_fenced(t, mu[h]), splat2(kRoundMagic));
+        const int tq0 = __viaddmin_s32_relu(__float_as_int(t.x), k.c1_add, k.c1_max);   // q2 - lo (lo == 0 here)
+        const int tq1 = __viaddmin_s32_relu(__float_as_int(t.y), k.c1_add, k.c1_max);
+        const float2 a = __ffma2_rn(splat2(k.a_scale), make_float2(__int2float_rn(tq0), __int2float_rn(tq1)), splat2(k.pa));
+        const float2 u = __fadd2_rn(fmul2_fenced(__fadd2_rn(a, rb), splat2(k.inv_scale)), splat2(kRoundMagic));
+        q[i] = __viaddmin_s32_relu(__float_as_int(u.x), k.c2_add, k.c2_max);                  // q - add_zp
+        q[i + 1] = __viaddmin_s32_relu(__float_as_int(u.y), k.c2_add, k.c2_max);
+      } else {
+        // the clamps (FMNMX) stand between the multiply and the magic-number adds: nothing here can be contracted
+        t = __fmul2_rn(t, mu[h]);
+        t = make_float2(fminf(fmaxf(t.x, k.lo_f), k.hi_f), fminf(fmaxf(t.y, k.lo_f), k.hi_f));
+        t = __fadd2_rn(__fadd2_rn(t, splat2(kRoundMagic)), splat2(-kRoundMagic));   // == float(q2 - zp2)
+        const float2 a = __ffma2_rn(splat2(k.a_scale), __fadd2_rn(t, splat2(k.zp_f)), splat2(k.pa));
+        const float2 s = __fadd2_rn(a, rb);
+        const float2 u = __fmul2_rn(make_float2(fmaxf(s.x, 0.0f), fmaxf(s.y, 0.0f)), splat2(k.inv_scale));
+        q[i] = __float2int_rn(u.x) + k.add_zp;
+        q[i + 1] = __float2int_rn(u.y) + k.add_zp;
+      }
+    }
+  }
+  uint4 o = make_uint4(pack4_sat_u8(q[0], q[1], q[2], q[3]), pack4_sat_u8(q[4], q[5], q[6], q[7]),
+                       pack4_sat_u8(q[8], q[9], q[10], q[11]), pack4_sat_u8(q[12], q[13], q[14], q[15]));
+  if (kFast) {     // bytes hold q - add_zp <= 255 - add_zp: the per-byte add cannot carry
+    o.x += k.zp4;
+    o.y += k.zp4;
+    o.z += k.zp4;
+    o.w += k.zp4;
+  }
+  return o;
+}
+
+#else   // IEVM_EXP_SCALAR_EPI: the scalar forms, one FADD / FMUL / FFMA per value (A/B build, scripts/build_ab.py)
+
 // 16 accumulators -> 16 requantised bytes (no residual).
 template <bool kFast>
 __device__ __forceinline__ uint4 epilogue16_i8(const uint32_t (&v)[16], const float* s_bd, const float* s_mu, int zp,
@@ -325,6 +432,7 @@ __device__ __forceinline__ uint4 epilogue16_i8_res(const uint32_t (&v)[16], cons
   }
   return o;
 }
+#endif   // IEVM_EXP_SCALAR_EPI
 
 template <bool kHasRes, bool kRelu>
 __device__ __forceinline__ void epilogue16_f16(const uint32_t (&v)[16], const float* s_bias, const __half* rp,
@@ -945,7 +1053,15 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
       rr[0] = rr[1] = make_uint4(0u, 0u, 0u, 0u);
       uint4 rq[2];                                // FP16: second half of a chunk's residual
       rq[0] = rq[1] = rr[0];
-      if (kResI8) rr[0] = load_res16_i8(p, m, valid, 0);
+      // INT8, at most four chunks: every residual chunk of the row is loaded before the accumulator wait (loading one
+      // chunk ahead leaves an L2 round trip exposed behind each chunk's arithmetic: 53 vs 49 us per layer-1 residual conv)
+      constexpr bool kResAll = kResI8 && kNch <= 4;
+      uint4 ra[kResAll ? kNch : 1];
+      if (kResAll) {
+#pragma unroll
+        for (int c = 0; c < (kResAll ? kNch : 1); ++c) ra[c] = load_res16_i8(p, m, valid, c * 16);
+      }
+      if (kResI8 && !kResAll) rr[0] = load_res16_i8(p, m, valid, 0);
       if (kResF16) load_res16_f16(p, m, valid, 0, rr[0], rq[0]);
       IEVM_TIMED_WAIT(tm_wait_a, &tfull_bar[acc], acc_phase, 0x400u | acc, p.stuck_flag);
       tc_fence_after();
@@ -959,10 +1075,11 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
           tmem_ld_wait();
           if (c + 1 < kNch) {
             tmem_ld_32x32b_x16(t_row + static_cast<uint32_t>((c + 1) * 16), vv[(c + 1) & 1]);
-            if (kResI8) rr[(c + 1) & 1] = load_res16_i8(p, m, valid, (c + 1) * 16);
+            if (kResI8 && !kResAll) rr[(c + 1) & 1] = load_res16_i8(p, m, valid, (c + 1) * 16);
             if (kResF16) load_res16_f16(p, m, valid, (c + 1) * 16, rr[(c + 1) & 1], rq[(c + 1) & 1]);
           }
-          epilogue_chunk<kDtype, kHasRes, false, kFs>(p, vv[c & 1], rr[c & 1], m, valid, c * 16, p.epc0, p.epc1, k, rq[c & 1]);
+          epilogue_chunk<kDtype, kHasRes, false, kFs>(p, vv[c & 1], kResAll ? ra[c < (kResAll ? kNch : 1) ? c : 0] : rr[c & 1],
+                                                     m, valid, c * 16, p.epc0, p.epc1, k, rq[c & 1]);
         }
       } else {
         // wide layers: the chunk loop stays a loop over chunk PAIRS (register budget); the tables are still read from

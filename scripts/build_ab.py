@@ -6,7 +6,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from ievm_b200 import _lib
 
 VARIANTS = {"halfk": ["IEVM_EXP_HALFK"], "interleave": ["IEVM_EXP_INTERLEAVE"],
-            "interleave_halfk": ["IEVM_EXP_INTERLEAVE", "IEVM_EXP_HALFK"]}
+            "interleave_halfk": ["IEVM_EXP_INTERLEAVE", "IEVM_EXP_HALFK"], "scalar_epi": ["IEVM_EXP_SCALAR_EPI"]}
 os.makedirs(os.path.join(_lib.ROOT, "ab"), exist_ok=True)
 for name in (sys.argv[1:] or VARIANTS):
     print(_lib.build(defines=VARIANTS[name], out=os.path.join(_lib.ROOT, "ab", f"lib_{name}.so")))

@@ -1,12 +1,14 @@
 // Micro-benchmark: per-SM issue rate of the instructions the requantisation epilogues are made of.
 // One CTA per SM, W warps, each warp runs N iterations of 16 independent chains of one op.
 // Prints cycles per warp-instruction per SMSP (lower = faster).   nvcc -arch=sm_100a -O3 pipes.cu -o pipes
+// The paired rows (FADD2 / FMUL2 / FFMA2) run chains of float2: one instruction does two lanes' work, so a paired op at the
+// scalar op's cycles per instruction halves the issue cost per value.
 #include <cstdio>
 #include <cstdint>
 #include <cuda_runtime.h>
 
-enum Op { I2F, F2I, FADD, FMUL, IADD, IMNMX, PRMT, I2IP, FMNMX, MIX_CUR, MIX_MAGIC, MIX_H1, ADDRELU_CUR, ADDRELU_NEW, NOPS };
-static const char* kNames[] = {"I2F", "F2I", "FADD", "FMUL", "IADD", "VIMNMX", "PRMT", "I2IP(cvt.pack)", "FMNMX",
+enum Op { I2F, F2I, FADD, FMUL, FFMA, FADD2, FMUL2, FFMA2, IADD, IMNMX, PRMT, I2IP, FMNMX, MIX_CUR, MIX_MAGIC, MIX_H1, ADDRELU_CUR, ADDRELU_NEW, NOPS };
+static const char* kNames[] = {"I2F", "F2I", "FADD", "FMUL", "FFMA", "FADD2", "FMUL2", "FFMA2", "IADD", "VIMNMX", "PRMT", "I2IP(cvt.pack)", "FMNMX",
                                "requant_current(6/val)", "requant_magic(8.75/val)", "requant_H1(I2F+magic round)",
                                "add_relu_current", "add_relu_new(magic final round)"};
 
@@ -14,8 +16,14 @@ template <int kOp>
 __global__ void bench(int iters, float fa, int ia, unsigned long long* out_cycles, int* sink) {
   int x[16];
   float f[16];
+  float2 g[16];
 #pragma unroll
-  for (int i = 0; i < 16; ++i) { x[i] = threadIdx.x * 17 + i * ia; f[i] = fa * (threadIdx.x + i); }
+  for (int i = 0; i < 16; ++i) {
+    x[i] = threadIdx.x * 17 + i * ia;
+    f[i] = fa * (threadIdx.x + i);
+    g[i] = make_float2(f[i], fa * (threadIdx.x + 2 * i));
+  }
+  const float2 fa2 = make_float2(fa, fa * fa);
   __syncthreads();
   const unsigned long long t0 = clock64();
   for (int it = 0; it < iters; ++it) {
@@ -25,6 +33,10 @@ __global__ void bench(int iters, float fa, int ia, unsigned long long* out_cycle
       else if (kOp == F2I) { x[i] = __float2int_rn(f[i]); f[i] = __int_as_float(x[i] | 0x3f800000); }
       else if (kOp == FADD) f[i] = __fadd_rn(f[i], fa);
       else if (kOp == FMUL) f[i] = __fmul_rn(f[i], fa);
+      else if (kOp == FFMA) f[i] = __fmaf_rn(f[i], fa, fa);
+      else if (kOp == FADD2) g[i] = __fadd2_rn(g[i], fa2);
+      else if (kOp == FMUL2) g[i] = __fmul2_rn(g[i], fa2);
+      else if (kOp == FFMA2) g[i] = __ffma2_rn(g[i], fa2, fa2);
       else if (kOp == IADD) x[i] = x[i] + ia;
       else if (kOp == IMNMX) x[i] = max(x[i], ia + i) ;
       else if (kOp == PRMT) x[i] = __byte_perm(x[i], ia, 0x4321);
@@ -56,7 +68,7 @@ __global__ void bench(int iters, float fa, int ia, unsigned long long* out_cycle
   const unsigned long long t1 = clock64();
   int s = 0;
 #pragma unroll
-  for (int i = 0; i < 16; ++i) s += x[i] + __float_as_int(f[i]);
+  for (int i = 0; i < 16; ++i) s += x[i] + __float_as_int(f[i]) + __float_as_int(g[i].x) + __float_as_int(g[i].y);
   if (s == 0x12345) *sink = s;
   if (threadIdx.x == 0 && blockIdx.x == 0) *out_cycles = t1 - t0;
 }
@@ -84,6 +96,10 @@ int main() {
     run<F2I>(warps, d_cyc, d_sink);
     run<FADD>(warps, d_cyc, d_sink);
     run<FMUL>(warps, d_cyc, d_sink);
+    run<FFMA>(warps, d_cyc, d_sink);
+    run<FADD2>(warps, d_cyc, d_sink);
+    run<FMUL2>(warps, d_cyc, d_sink);
+    run<FFMA2>(warps, d_cyc, d_sink);
     run<IADD>(warps, d_cyc, d_sink);
     run<IMNMX>(warps, d_cyc, d_sink);
     run<PRMT>(warps, d_cyc, d_sink);
