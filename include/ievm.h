@@ -213,8 +213,11 @@ int ievm_debug_conv_acc(ievm_handle* h, int layer, int n, int32_t* host_out, uin
 
 /* Runs ONLY the fused front end (quantize + stem + ReLU + max-pool, frontend_v2.cuh) on the device batch
  * x_dev and copies the pooled tensor [n][ph][pw][c_pitch] (u8 / f16) to pooled_host; when acc_host is not
- * NULL also the stem's zero-point-corrected accumulators [n][ho][wo][c_pitch] (int32; fp32 bits for F16). */
-int ievm_debug_frontend(ievm_handle* h, const void* x_dev, int n, void* pooled_host, uint64_t pooled_bytes,
+ * NULL also the stem's zero-point-corrected accumulators [n][ho][wo][c_pitch] (int32; fp32 bits for F16).
+ * in_mode 0: x_dev is the engine's native input (f32 / f16 NCHW); 1: decoded 8-bit images, u8 [n][in_h][in_w][3]
+ * through the lookup table of ievm_set_input_lut (INT8 engines).  Without acc_host the kernel the forward would
+ * launch for that input runs. */
+int ievm_debug_frontend(ievm_handle* h, const void* x_dev, int in_mode, int n, void* pooled_host, uint64_t pooled_bytes,
                         int32_t* acc_host, uint64_t acc_bytes);
 
 /* Diagnostic: issue ONE im2col-mode TMA load (128 pixels x kc_bytes channels of a u8 NHWC tensor

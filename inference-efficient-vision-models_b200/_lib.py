@@ -136,7 +136,7 @@ def load():
     lib.ievm_debug_resize.restype = C.c_int
     lib.ievm_count_correct.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
     lib.ievm_count_correct.restype = C.c_int
-    lib.ievm_debug_frontend.argtypes = [H, C.c_void_p, C.c_int, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64]
+    lib.ievm_debug_frontend.argtypes = [H, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64]
     lib.ievm_debug_frontend.restype = C.c_int
     lib.ievm_profile_read.argtypes = [H, C.c_int, C.c_void_p, C.c_void_p]
     lib.ievm_profile_read.restype = C.c_int

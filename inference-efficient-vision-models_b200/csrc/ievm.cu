@@ -1432,7 +1432,8 @@ int launch_frontend2(ievm_handle* h, const void* x, int n, cudaStream_t s, int32
   const int grid = std::min(n * fp.ph, h->num_sms);       // contiguous ranges of pooled rows (frontend_v2.cuh: F2Walk)
   if (dump_acc != nullptr) {
     // debug instantiations (ievm_debug_frontend): the general rounding form, accumulators written out
-    if (i8) frontend2_kernel<kDtypeI8, 0, false, true><<<grid, kF2Threads, F2Cfg<kDtypeI8>::kSmemBytes, s>>>(tmap, fp);
+    if (u8_input) frontend2_kernel<kDtypeI8, 1, false, true><<<grid, kF2Threads, F2Cfg<kDtypeI8, 1>::kSmemBytes, s>>>(tmap, fp);
+    else if (i8) frontend2_kernel<kDtypeI8, 0, false, true><<<grid, kF2Threads, F2Cfg<kDtypeI8>::kSmemBytes, s>>>(tmap, fp);
     else frontend2_kernel<kDtypeF16, 0, false, true><<<grid, kF2Threads, F2Cfg<kDtypeF16>::kSmemBytes, s>>>(tmap, fp);
   } else if (u8_input && fp.fast_round) frontend2_kernel<kDtypeI8, 1, true><<<grid, kF2Threads, F2Cfg<kDtypeI8, 1>::kSmemBytes, s>>>(tmap, fp);
   else if (u8_input) frontend2_kernel<kDtypeI8, 1><<<grid, kF2Threads, F2Cfg<kDtypeI8, 1>::kSmemBytes, s>>>(tmap, fp);
@@ -1860,6 +1861,10 @@ int ievm_create(const ievm_net_desc* nd, int device, int max_batch, ievm_handle*
              ? cudaFuncSetAttribute(frontend2_kernel<kDtypeI8, 0, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)F2Cfg<kDtypeI8>::kSmemBytes)
              : cudaFuncSetAttribute(frontend2_kernel<kDtypeF16, 0, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)F2Cfg<kDtypeF16>::kSmemBytes)) != cudaSuccess)
       rc = fail(IEVM_ERR_CUDA, "cudaFuncSetAttribute(frontend2_kernel, debug instantiation) failed");
+    else if (h->dtype == IEVM_DTYPE_I8 &&
+             cudaFuncSetAttribute(frontend2_kernel<kDtypeI8, 1, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  (int)F2Cfg<kDtypeI8, 1>::kSmemBytes) != cudaSuccess)
+      rc = fail(IEVM_ERR_CUDA, "cudaFuncSetAttribute(frontend2_kernel, u8 debug instantiation) failed");
   }
   if (rc == IEVM_OK && h->front2_ok) {
     const cudaError_t e = h->dtype == IEVM_DTYPE_I8
@@ -2476,10 +2481,14 @@ int ievm_debug_conv_acc(ievm_handle* h, int layer, int n, int32_t* host_out, uin
   return rc;
 }
 
-int ievm_debug_frontend(ievm_handle* h, const void* x_dev, int n, void* pooled_host, uint64_t pooled_bytes,
+int ievm_debug_frontend(ievm_handle* h, const void* x_dev, int in_mode, int n, void* pooled_host, uint64_t pooled_bytes,
                         int32_t* acc_host, uint64_t acc_bytes) {
-  if (!h || !x_dev || !pooled_host || n <= 0 || n > h->max_batch) return fail(IEVM_ERR_BAD_ARG, "debug_frontend: bad arguments");
+  if (!h || !x_dev || !pooled_host || n <= 0 || n > h->max_batch || (in_mode != kInNative && in_mode != kInU8))
+    return fail(IEVM_ERR_BAD_ARG, "debug_frontend: bad arguments");
   if (!h->front2_ok) return fail(IEVM_ERR_UNSUPPORTED, "this network's front end does not fit the fused v2 kernel");
+  const bool u8_input = in_mode == kInU8;
+  if (u8_input && h->dtype != IEVM_DTYPE_I8) return fail(IEVM_ERR_UNSUPPORTED, "8-bit image input belongs to INT8 engines");
+  if (u8_input && h->lut_dev == nullptr) return fail(IEVM_ERR_BAD_ARG, "call ievm_set_input_lut before debug_frontend on u8 images");
   const LayerPlan& Ls = h->layers[0];
   const LayerPlan& Lp = h->layers[1];
   const size_t pooled = static_cast<size_t>(n) * Lp.ho * Lp.wo * Ls.cout_pad * h->elem;
@@ -2489,7 +2498,7 @@ int ievm_debug_frontend(ievm_handle* h, const void* x_dev, int n, void* pooled_h
   int32_t* dacc = nullptr;
   if (acc_host) CUDA_TRY(cudaMalloc(reinterpret_cast<void**>(&dacc), acc));
   cudaDeviceSynchronize();                  // parity hook: earlier work on other streams is done
-  int rc = launch_frontend2(h, x_dev, n, h->own_stream, dacc);
+  int rc = launch_frontend2(h, x_dev, n, h->own_stream, dacc, u8_input);
   if (rc == IEVM_OK) rc = check_stuck(h, cudaStreamSynchronize(h->own_stream), "debug_frontend");
   if (rc == IEVM_OK && cudaMemcpy(pooled_host, tensor_ptr(h, Lp.d.out_tensor), pooled, cudaMemcpyDeviceToHost) != cudaSuccess)
     rc = fail(IEVM_ERR_CUDA, "pooled tensor copy failed");

@@ -160,7 +160,8 @@ class _B200Engine(nn.Module):
         """Enqueue ``model(images)`` for a CPU batch and return at once (``ievm_submit_*_host``): the H2D copy of this
         batch overlaps the forward of the previous one.  ``images`` is what ``forward`` accepts on the CPU (pinned
         memory makes the copy asynchronous) or, for INT8 engines, decoded uint8 ``[N, h, w, 3]`` images.  At most two
-        batches are in flight; ``.result()`` of the returned object waits for this one's logits (a CPU tensor)."""
+        batches are in flight: a third call first settles the oldest one, whose ``.result()`` then returns at once.
+        ``.result()`` of the returned object waits for this one's logits (a CPU tensor)."""
         if images.is_cuda:
             raise ValueError("submit() is the host-buffer path; call the engine directly with CUDA tensors")
         n = int(images.shape[0])
@@ -178,12 +179,21 @@ class _B200Engine(nn.Module):
         if not hasattr(self, "_out_ring"):       # two pinned logits buffers, one per pipeline slot
             self._out_ring = [torch.empty((self.max_batch, self.net.num_classes), dtype=self._torch_dtype).pin_memory()
                               for _ in range(2)]
+            self._out_owner = [None, None]
             self._out_next = 0
-        out = self._out_ring[self._out_next]
+        k = self._out_next
+        # The call that last used this buffer may not have been read yet: settle it (copy its logits out) before this
+        # call's D2H overwrites them.  The C submit waits for that call's slot anyway, so this adds no synchronisation.
+        if self._out_owner[k] is not None:
+            self._out_owner[k].result()
+            self._out_owner[k] = None
+        out = self._out_ring[k]
         self._out_next ^= 1
         ticket = C.c_int64(-1)
         _lib.check(fn(self._handle, x.data_ptr(), n, out.data_ptr(), C.byref(ticket)), "ievm_submit_host")
-        return PendingLogits(self, int(ticket.value), out, n, x)
+        pending = PendingLogits(self, int(ticket.value), out, n, x)
+        self._out_owner[k] = pending
+        return pending
 
     def _submit_u8(self, x: torch.Tensor):
         raise TypeError("uint8 image input belongs to the INT8 engine")
@@ -261,17 +271,23 @@ class _B200Engine(nn.Module):
         raise KeyError(layer_name)
 
     def debug_frontend(self, images: torch.Tensor, want_acc: bool = True):
-        """Run only the fused front end (quantize + stem + ReLU + max-pool) on a CUDA batch.  Returns
-        (pooled NCHW over real channels, stem accumulators NCHW or None)."""
+        """Run only the fused front end (quantize + stem + ReLU + max-pool) on a CUDA batch: the engine's native input,
+        or decoded uint8 ``[N, in_h, in_w, 3]`` images through the lookup table of ``set_input_transform`` (INT8).
+        Returns (pooled NCHW over real channels, stem accumulators NCHW or None)."""
         stem, pool = self.net.layers[0], self.net.layers[1]
         n = int(images.shape[0])
+        u8 = images.dtype == torch.uint8
+        if u8 and (images.dim() != 4 or tuple(images.shape[1:]) != (self.net.in_h, self.net.in_w, 3)):
+            raise ValueError(f"expected uint8 [N,{self.net.in_h},{self.net.in_w},3], got {tuple(images.shape)}")
+        if u8 and getattr(self, "_lut", None) is None:
+            raise ValueError("debug_frontend on uint8 images needs set_input_transform() first")
         _, ho, wo, c, pitch, elem = self.tensor_shape(stem.out_tensor)
         _, ph, pw, _, _, _ = self.tensor_shape(pool.out_tensor)
         dt = np.uint8 if elem == 1 else np.float16
         pooled = np.empty((n, ph, pw, pitch), dtype=dt)
         acc = np.empty((n, ho, wo, pitch), dtype=np.int32) if want_acc else None
         x = images.contiguous()
-        _lib.check(self._lib.ievm_debug_frontend(self._handle, x.data_ptr(), n, pooled.ctypes.data, pooled.nbytes,
+        _lib.check(self._lib.ievm_debug_frontend(self._handle, x.data_ptr(), int(u8), n, pooled.ctypes.data, pooled.nbytes,
                                                  acc.ctypes.data if want_acc else None, acc.nbytes if want_acc else 0),
                    "debug_frontend")
         pooled = np.ascontiguousarray(pooled[..., :c].transpose(0, 3, 1, 2))

@@ -6,6 +6,17 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 _CACHE = {}
 
+# Decoded-image source sizes (h, w) the GPU resize is checked at, against Pillow and the oracle's restatement
+RESIZE_SOURCES = [
+    (200, 200), (300, 260), (97, 131),
+    (224, 300), (300, 224), (224, 97), (97, 224),      # one axis only: the horizontal pass alone writes the output, or
+                                                       # the vertical pass alone reads the caller's buffer
+    (223, 225), (225, 223),                            # near identity
+    (1, 1), (1, 224), (224, 1), (2, 3), (7, 5),        # tiny sources
+    (17, 600), (600, 17),                              # upscale one axis, downscale the other
+    (1080, 1920), (3000, 4000),                        # strong downscales: up to 2 * ceil(src / 224) + 1 taps
+]
+
 
 def cached_quantized(widths):
     """Converted INT8 module for `widths` (PTQ takes a few seconds; share it across tests)."""

@@ -184,6 +184,35 @@ def test_submit_wait_equals_the_synchronous_call():
     e16.close()
 
 
+@pytest.mark.parametrize("kind", ["f32", "u8_resize", "fp16"])
+def test_submit_results_read_out_of_order_are_not_overwritten(kind):
+    """Three submits before any result: the third reuses the first call's pinned logits buffer.  Each result, read in
+    the order 3, 2, 1, must still be its own batch's logits (the first call is settled before its buffer is reused)."""
+    import ievm_b200
+    sizes = (16, 3, 9)
+    if kind == "fp16":
+        eng, _ = _fp16_engine_and_module(mf.PRUNED_WIDTHS, 16)
+        xs = [mf.synthetic_images(n, seed=110 + i).half().pin_memory() for i, n in enumerate(sizes)]
+        want = [eng(x.cuda()).cpu() for x in xs]
+    else:
+        eng = ievm_b200.B200QuantizedResNet.from_converted(cached_quantized(mf.PRUNED_WIDTHS), max_batch=16)
+        if kind == "f32":
+            xs = [mf.synthetic_images(n, seed=110 + i).pin_memory() for i, n in enumerate(sizes)]
+            want = [eng(x.cuda()).cpu() for x in xs]
+        else:
+            g = torch.Generator().manual_seed(110)
+            xs = [torch.randint(0, 256, (n, 200, 200, 3), dtype=torch.uint8, generator=g).pin_memory() for n in sizes]
+            want = [eng.forward_u8(x.cuda()).cpu() for x in xs]
+    pend = [eng.submit(x) for x in xs]
+    got = [None] * 3
+    for i in (2, 1, 0):
+        got[i] = pend[i].result()
+    for i, (g_, w) in enumerate(zip(got, want)):
+        assert g_.shape == w.shape and torch.equal(g_, w), \
+            f"{kind}: result of submit {i + 1} (batch {sizes[i]}) is not its own batch's logits"
+    eng.close()
+
+
 def test_evaluate_accuracy_over_cpu_batches_is_pipelined_and_exact():
     """The reference's loop (engines.py:52-63) over CPU batches: same accuracy as the reference module on the CPU."""
     import ievm_b200

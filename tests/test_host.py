@@ -12,7 +12,7 @@ import torch
 import ievm_b200
 from ievm_b200 import _lib
 from oracle import model_factory as mf
-from ievm_testutil import ROOT, cached_quantized
+from ievm_testutil import RESIZE_SOURCES, ROOT, cached_quantized
 
 
 def test_library_builds_and_exports_every_declared_symbol():
@@ -123,7 +123,8 @@ def test_input_lut_equals_the_reference_transform_pipeline():
 def test_resize_tables_equal_the_oracle_restatement():
     """The product's Pillow coefficient tables (host side of ievm_set_resize) against the oracle's restatement."""
     from oracle.pil_resize import precompute_coeffs
-    for src in (200, 224, 300, 97, 31, 500):
+    sizes = {200, 224, 300, 97, 31, 500} | {v for hw in RESIZE_SOURCES for v in hw}
+    for src in sorted(sizes):
         b, k = ievm_b200.pil_bilinear_coeffs(src, 224)
         bo, ko = precompute_coeffs(src, 224)
         assert np.array_equal(b, bo) and np.array_equal(k, ko), src
